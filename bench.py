@@ -2,6 +2,7 @@
 """bench.py -- edges/sec per GCN layer (128-d feat) on synthetic power-law graphs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg5|cfg3|cfg4]
+                    [--dump-outputs DIR]
 
 One "step" = one GCN-layer aggregation over the whole graph: ``send_recv(sum)`` with both
 degree-norm scalings (reference pgl/nn/conv.py:242-250 around graph.py:860), i.e. the SpMM the
@@ -24,6 +25,10 @@ Prints ONE JSON line (rank 0).  Keys follow the driver contract; additionally
 
 ``--config cfg3`` (GATConv on RMAT 1M/10M) and ``--config cfg4`` (3-layer GraphSAGE on a products-shape
 graph) time BASELINE.json configs[2] and configs[3] with their own roofline models.
+
+``--dump-outputs DIR`` writes what the timed path returned in its last timed step to DIR/<name>.npy
+(float32, one row per output row, the row numbers in DIR/<name>_rows.npy; see dump_outputs), so that two
+builds run with the same arguments -- hence the same seeded inputs -- can be compared output for output.
 """
 import argparse
 import ctypes
@@ -37,9 +42,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the package is imported from the tree, which bench.py leaves as it found it
 
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 PARITY_TOL = 1e-4           # north_star: "correctness matching reference PGL within 1e-4 relative"
+DUMP_BYTES = 48 << 20       # --dump-outputs: bytes of all files of one run together (every rank included)
+DUMP_SEED = 0
 
 
 def parse():
@@ -63,7 +71,13 @@ def parse():
     ap.add_argument("--partition", default="block", choices=["block", "metis"])
     ap.add_argument("--halo", default=os.environ.get("PGLB_HALO_MODE", "p2p"), choices=["nccl", "p2p"])
     ap.add_argument("--overlap", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float32; a fixed seeded sample "
+                         "of the rows when the output is larger than %d MiB)" % (DUMP_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def host_threads():
@@ -206,8 +220,12 @@ def _i64(v):
 
 
 def _load_oracle_c():
+    """The oracle's C library as build() left it.  bench.py writes nothing into the tree (it may be read-only):
+    a missing or out-of-date library is compiled into a temporary directory instead."""
+    import tempfile
     from oracle import build as obuild
-    return ctypes.CDLL(obuild.build_oracle_c())
+    with tempfile.TemporaryDirectory(prefix="pglb_oracle_") as tmp:
+        return ctypes.CDLL(obuild.build_oracle_c(out=os.path.join(tmp, "liboracle_c.so")))
 
 
 class CpuGcn(object):
@@ -344,6 +362,8 @@ def main_reference(args):
         t, info = prob.run(x_np, norm_np, threads)
         if i >= args.warmup:
             vals.append(prob.e_s / t)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"gcn_aggregate": prob.out})
     v = float(np.median(vals))
     line = {
         "impl": "reference", "metric": "edges/sec per GCN layer (128-d feat)", "value": v,
@@ -377,22 +397,54 @@ def _ev(torch):
 
 def timed_steps(torch, step, steps, dist=None):
     """EXACTLY `steps` calls bracketed by synchronize (+ barrier) on both sides; per-step CUDA events on the
-    launching stream.  Returns (total_ms, sorted per-step ms)."""
+    launching stream.  Returns (total_ms, sorted per-step ms, what the last call returned).  Only the last
+    call's result is kept, so earlier results are freed as soon as their call returns."""
     evs = [(_ev(torch), _ev(torch)) for _ in range(steps)]
+    last = None
     torch.cuda.synchronize()
     if dist is not None:
         dist.barrier()
     b0, b1 = _ev(torch), _ev(torch)
     b0.record()
-    for a, b in evs:
+    for i, (a, b) in enumerate(evs):
         a.record()
-        step()
+        if i + 1 < steps:
+            step()
+        else:
+            last = step()
         b.record()
     b1.record()
     torch.cuda.synchronize()
     if dist is not None:
         dist.barrier()
-    return b0.elapsed_time(b1), sorted(a.elapsed_time(b) for a, b in evs)
+    return b0.elapsed_time(b1), sorted(a.elapsed_time(b) for a, b in evs), last
+
+
+def dump_outputs(path, outputs, rank=0, world=1):
+    """--dump-outputs: every array in `outputs` ({name: torch tensor or numpy array}) -> path/<name>.npy as float32
+    rows [k, a[0].size], and path/<name>_rows.npy (float64 [k]): which rows of `a` they are (names suffixed with
+    the rank when several ranks write).  An array larger than its share of DUMP_BYTES is stored as a fixed sample
+    of its rows (DUMP_SEED, ascending row order): the same rows in every run with the same arguments.  Row i of
+    the single-GPU cfg5 output is graph row i, in both arms; the reference arm's output holds only the rows it
+    timed (dst < n_s, all of them when config.same_workload_as_gpu_arm)."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // (world * len(outputs))
+    for name, a in outputs.items():
+        rows = a.reshape(a.shape[0], -1)
+        k = min(rows.shape[0], max(1, share // (4 * max(1, rows.shape[1]) + 8)))
+        idx = np.arange(rows.shape[0])
+        if k < rows.shape[0]:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rows.shape[0], k, replace=False))
+            if isinstance(rows, np.ndarray):
+                rows = rows[idx]
+            else:
+                import torch
+                rows = rows[torch.from_numpy(idx).to(rows.device)]
+        if not isinstance(rows, np.ndarray):
+            rows = rows.float().cpu().numpy()
+        fname = name if world == 1 else "%s_rank%d" % (name, rank)
+        np.save(os.path.join(path, fname + ".npy"), np.ascontiguousarray(rows, dtype=np.float32))
+        np.save(os.path.join(path, fname + "_rows.npy"), idx.astype(np.float64))
 
 
 def read_traffic(key):
@@ -552,9 +604,11 @@ def bench_gcn(args, torch, dist, pgl, ops, GF, dev, world, rank):
     sampler = ClockSampler(dev.index)
     sampler.start()
     l0 = ops.launch_count()
-    total_ms, per = timed_steps(torch, step, args.steps, dist)
+    total_ms, per, last = timed_steps(torch, step, args.steps, dist)
     launches = ops.launch_count() - l0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"gcn_aggregate": last}, rank, world)
     kern_ms = float(np.mean(per))
     b_alg = algorithmic_bytes(n_loc, e_loc, dl)    # this rank's kernel: its edges, its rows, its columns
     achieved = b_alg / (kern_ms * 1e-3) / 1e9
@@ -916,9 +970,12 @@ def bench_row_sharded(args, torch, dist, pgl, dev, world, rank):
     sampler = ClockSampler(dev.index)
     sampler.start()
     l0 = ops.launch_count()
-    total_ms, per = timed_steps(torch, step, args.steps, dist)
+    total_ms, per, last = timed_steps(torch, step, args.steps, dist)
     launches = ops.launch_count() - l0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"gcn_aggregate": last}, rank, world)
+    del last
     ms = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_step = float(ms.item()) / args.steps
@@ -1010,9 +1067,12 @@ def bench_gat(args, torch, pgl, ops, GF, dev):
         sampler = ClockSampler(dev.index)
         sampler.start()
         l0 = ops.launch_count()
-        total_ms, per = timed_steps(torch, step, args.steps)
+        total_ms, per, last = timed_steps(torch, step, args.steps)
         launches = ops.launch_count() - l0
         clocks = sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"gat_aggregate": last})
+        del last
         for _ in range(3):
             conv(g, x)
         torch.cuda.synchronize()
@@ -1165,16 +1225,19 @@ def bench_sage(args, torch, dist, pgl, ops, GF, dev, world, rank):
         sampler = ClockSampler(dev.index)
         sampler.start()
         l0 = ops.launch_count()
-        total_ms, per = timed_steps(torch, forward, args.steps)
+        total_ms, per, last = timed_steps(torch, forward, args.steps)
         launches = ops.launch_count() - l0
         clocks = sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"sage_forward": last})
+        del last
         h = x
         for i, conv in enumerate(layers):
             d = dims[i]
             agg = lambda: g.send_recv(h, "mean")   # noqa: E731
             for _ in range(3):
                 agg()
-            t_ms, p_ = timed_steps(torch, agg, 5)
+            t_ms, p_, _ = timed_steps(torch, agg, 5)
             b_alg = e * (4 * d + 8) + n * 4 * d + (n + 1) * 8
             per_layer.append({"in": d, "out": dims[i + 1], "aggregation_ms": t_ms / 5,
                               "agg_alg_GBs": b_alg / (t_ms / 5) / 1e6,
@@ -1252,9 +1315,12 @@ def bench_sage_sharded(args, torch, dist, pgl, ops, dev, world, rank, edges, x, 
         sampler = ClockSampler(dev.index)
         sampler.start()
         l0 = ops.launch_count()
-        total_ms, per = timed_steps(torch, forward, args.steps, dist)
+        total_ms, per, last = timed_steps(torch, forward, args.steps, dist)
         launches = ops.launch_count() - l0
         clocks = sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"sage_forward": last}, rank, world)
+        del last
     t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = float(t.item()) / args.steps

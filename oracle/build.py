@@ -8,7 +8,8 @@
   only into ``oracle/_ref/`` (git-ignored, not gpurun-ignored).  Mirrors the source/include
   lists of ``/root/reference/setup.py:82-117`` without running the reference's build
   system.  No reference source is copied into the repository; the generated
-  ``graph_kernel.cpp`` is an intermediate inside ``oracle/_ref/build``.
+  ``graph_kernel.cpp`` is an intermediate inside ``oracle/_ref/build``.  The METIS objects
+  are also linked alone into ``oracle/_ref/libmetis_i64.so``.
 
 ``load_ref_graph_kernel()`` imports the built module directly (bypassing
 ``pgl/__init__.py:21`` which needs paddle) and returns None when it has not been built
@@ -44,11 +45,13 @@ def oracle_c_path():
     return os.path.join(HERE, "liboracle_c.so")
 
 
-def build_oracle_c(force=False):
+def build_oracle_c(force=False, out=None):
+    """An up-to-date oracle/liboracle_c.so is reused; otherwise gcc writes the library to `out`
+    (default: oracle/liboracle_c.so)."""
     src = os.path.join(HERE, "oracle_c.c")
-    out = oracle_c_path()
-    if not force and _newer(out, [src]):
-        return out
+    if not force and _newer(oracle_c_path(), [src]):
+        return oracle_c_path()
+    out = out or oracle_c_path()
     _run(["gcc", "-O3", "-march=native", "-fopenmp", "-fPIC", "-shared", "-std=c11",
           "-o", out, src])
     return out
@@ -59,13 +62,19 @@ def ref_so_path():
     return os.path.join(REF_OUT, "graph_kernel" + suffix)
 
 
+def ref_metis_path():
+    return os.path.join(REF_OUT, "libmetis_i64.so")
+
+
 def build_ref(force=False, jobs=8):
-    """Compile the reference's graph_kernel.pyx + METIS into oracle/_ref/."""
+    """Compile the reference's graph_kernel.pyx + METIS into oracle/_ref/, and link the METIS objects
+    alone into oracle/_ref/libmetis_i64.so (what pgl_b200/build.py:build_metis makes from the same
+    sources with the same flags) for the METIS tests where the package's own copy cannot be built."""
     pyx = os.path.join(REF, "pgl", "graph_kernel.pyx")
     out = ref_so_path()
     if not os.path.exists(pyx):
         return out if os.path.exists(out) else None
-    if not force and os.path.exists(out):
+    if not force and os.path.exists(out) and os.path.exists(ref_metis_path()):
         return out
     import numpy
 
@@ -105,6 +114,8 @@ def build_ref(force=False, jobs=8):
     o_main = os.path.join(bdir, "graph_kernel.o")
     _run(["g++", "-O2", "-fPIC", "-w", "-std=c++11", "-c", cpp, "-o", o_main] + incs)
     _run(["g++", "-shared", "-o", out, o_main] + objs + ["-lm"])
+    metis_objs = [o for o in objs if os.path.basename(o).startswith(("GKlib_", "libmetis_"))]
+    _run(["gcc", "-shared", "-o", ref_metis_path()] + metis_objs + ["-lm"])
     return out
 
 

@@ -19,8 +19,10 @@ def pytest_configure(config):
         __graft_entry__.load_builder().build_all()
     from oracle import build as obuild
     obuild.build_oracle_c()
-    if os.path.isdir("/root/reference"):
-        obuild.build_ref()
+    # METIS for the METIS tests: the package's own copy, else the one build() links into oracle/_ref
+    import __graft_entry__
+    if not os.path.exists(__graft_entry__.load_builder().METIS_LIB) and os.path.exists(obuild.ref_metis_path()):
+        os.environ.setdefault("PGLB_LIBMETIS", obuild.ref_metis_path())
 
 
 def pytest_collection_modifyitems(config, items):

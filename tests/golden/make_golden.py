@@ -10,6 +10,11 @@ Two kinds of fixture:
    ``pgl.graph_kernel`` (built by oracle/build.py into oracle/_ref/) on seeded inputs:
    ``build_index`` (pgl/graph_kernel.pyx:59-88) and ``metis_partition``
    (pgl/graph_kernel.pyx:434-472, K-way, as pgl/partition.py:83-90 calls it).
+3. ``ref_graph_kernel.npz`` -- outputs of the same compiled module for the seeded inputs the
+   relabelling and index tests draw (``map_nodes`` / ``map_edges`` / ``build_index``), plus a fixed
+   set of small edge lists (empty, one node, duplicates, self loops, ids beyond the largest one)
+   with their ``build_index`` results, so those tests compare with the reference everywhere.
+   ``python tests/golden/make_golden.py graph_kernel`` rewrites only this file.
 """
 import json
 import os
@@ -115,11 +120,72 @@ def power_law_edges(n, e, seed):
     return p[s].astype(np.int64), p[d].astype(np.int64)
 
 
+BUILD_INDEX_FIELDS = ("degree", "sorted_v", "sorted_u", "sorted_eid", "indptr")
+INDEX_CASES = 80
+
+
+def index_cases(seed=17):
+    """Small (u, v, num_nodes) edge lists shaped like tests/test_property_index.py draws them."""
+    rng = np.random.default_rng(seed)
+    cases = [(np.zeros(0, np.int64), np.zeros(0, np.int64), 1), (np.zeros(0, np.int64), np.zeros(0, np.int64), 6),
+             (np.zeros(3, np.int64), np.zeros(3, np.int64), 1)]
+    while len(cases) < INDEX_CASES:
+        n = int(rng.integers(1, 41))
+        e = int(rng.integers(0, 121))
+        u = rng.integers(0, n, e).astype(np.int64)
+        v = rng.integers(0, n, e).astype(np.int64)
+        cases.append((u, v, n + int(rng.integers(0, 6))))
+    return cases
+
+
+def graph_kernel_fixtures(gk):
+    """Every input is stored next to the reference's output on it: the tests read both."""
+    out = {}
+    # map_nodes / map_edges with the {old id: position} dict: tests/test_host_logic.py ("relabel") and
+    # tests/test_gpu_localgraph.py ("localgraph")
+    for name, seed, ids, n_old, n_nodes, n_edges, n_eid in (("relabel", 3, 50, 20, 30, 40, 15),
+                                                            ("localgraph", 401, 5000, 2000, 3000, 4000, 1500)):
+        rng = np.random.default_rng(seed)
+        old = rng.permutation(ids)[:n_old].astype(np.int64)
+        nodes = rng.choice(old, n_nodes)
+        edges = rng.choice(old, (n_edges, 2)).astype(np.int64)
+        eid = rng.integers(0, n_edges, n_eid).astype(np.int64)
+        reindex = {int(o): i for i, o in enumerate(old)}
+        out.update({name + "_old": old, name + "_nodes": nodes, name + "_edges": edges, name + "_eid": eid,
+                    name + "_map_nodes": np.asarray(gk.map_nodes(nodes, reindex)),
+                    name + "_map_edges": np.asarray(gk.map_edges(eid, edges, reindex))})
+    # pgl.sampling.subgraph's renumbering of the edges inside `nodes` (tests/test_host_logic.py)
+    rng = np.random.default_rng(0)
+    edges = rng.integers(0, 30, (60, 2)).astype(np.int64)
+    nodes = rng.permutation(30)[:20].astype(np.int64)
+    eid = np.flatnonzero(np.isin(edges[:, 0], nodes) & np.isin(edges[:, 1], nodes))
+    reindex = {int(v): i for i, v in enumerate(nodes)}
+    out["subgraph_edges"], out["subgraph_nodes"] = edges, nodes
+    out["subgraph_map_edges"] = np.asarray(gk.map_edges(np.arange(len(eid), dtype=np.int64), edges[eid], reindex))
+
+    def index_case(name, u, v, n):
+        out[name + "_u"], out[name + "_v"], out[name + "_n"] = u, v, np.int64(n)
+        for f, a in zip(BUILD_INDEX_FIELDS, gk.build_index(u, v, n)):
+            out[name + "_" + f] = np.asarray(a)
+
+    # build_index: three seeded edge lists (tests/test_oracle_golden.py) and the small cases
+    # (tests/test_property_index.py)
+    rng = np.random.default_rng(5)
+    for i, (n, e) in enumerate(((1, 0), (3, 10), (500, 5000))):
+        index_case("seeded%d" % i, rng.integers(0, n, e).astype(np.int64), rng.integers(0, n, e).astype(np.int64), n)
+    for i, (u, v, n) in enumerate(index_cases()):
+        index_case("case%02d" % i, u, v, n)
+    np.savez_compressed(os.path.join(HERE, "ref_graph_kernel.npz"), **out)
+
+
 def main():
     gk = obuild.load_ref_graph_kernel()
     if gk is None:
         obuild.build_ref()
         gk = obuild.load_ref_graph_kernel()
+    graph_kernel_fixtures(gk)
+    if sys.argv[1:] == ["graph_kernel"]:
+        return
     with open(os.path.join(HERE, "kat.json"), "w") as f:
         json.dump(kats(), f, indent=1)
 
