@@ -308,6 +308,57 @@ int pglb_reindex_graph(const int64_t *x, int64_t n, const int64_t *neighbors, co
                        int64_t m, int64_t *table, int64_t *reindex_src, int64_t *reindex_dst,
                        int64_t *out_nodes, int64_t *num_out, void *ws, size_t ws_bytes, void *stream);
 
+/* ------------------------------------------------------------------------------------
+ * Random walks and skip-gram pairs (csrc/walk.cu): pgl.sampling.random_walk / node2vec_walk /
+ * node2vec_walk_plus (pgl/sampling/walk.py:23-183, the per-step pgl/graph_kernel.pyx:142-224) and
+ * graph_kernel.skip_gram_gen_pair (pgl/graph_kernel.pyx:343-364) over a whole batch of walks.
+ *
+ * indptr[N+1], cols[E]: the successor CSR with every row's columns in ascending order.
+ * out[n, ldo] (ldo >= steps + 1): out[i, 0] = nodes[i], out[i, t+1] = the node reached by step t; a walk
+ * ends at the first node without successors and the rest of its row is -1.
+ *
+ * RNG, a pure function of (seed, i) whatever the launch geometry (all arithmetic mod 2^64):
+ *   mix64(z):  z += 0x9e3779b97f4a7c15; z = (z ^ z >> 30) * 0xbf58476d1ce4e5b9;
+ *              z = (z ^ z >> 27) * 0x94d049bb133111eb; return z ^ z >> 31
+ *   word(t, k) = mix64(mix64(seed ^ mix64(i)) + PGLB_WALK_WORDS_PER_STEP * t + k)
+ * Step t from node c with d > 0 successors cols[s .. s+d):
+ *   uniform mode, and step 0 of every mode: next = cols[s + umul64hi(word(t, 0), d)]
+ *   node2vec / node2vec+, t >= 1: the weight class of a candidate x is 0 when x is the previous node,
+ *     1 when x is in the seen set (node2vec: successors of the previous node; node2vec+: successors of
+ *     every earlier node of the walk), 2 otherwise.  With w = (1/p, 1, 1/q), M = max(w) (double):
+ *       T[c] = max(1, floor(w[c] / M * 2^32))
+ *     draw k = 0 .. PGLB_WALK_MAX_REJECT-1: x = cols[s + umul64hi(word(t, 2k), d)], accepted when
+ *       (word(t, 2k+1) >> 32) < T[class(x)];
+ *     when no draw is accepted: S = sum over the row's slots j of T[class(cols[s+j])],
+ *       r = umul64hi(word(t, 2 PGLB_WALK_MAX_REJECT), S), next = cols[s + first j whose inclusive prefix
+ *       sum of T exceeds r]  (exact inverse CDF; on the device one warp per such step).
+ * Both entries produce the same walks bit for bit.
+ * ---------------------------------------------------------------------------------- */
+#define PGLB_WALK_UNIFORM 0
+#define PGLB_WALK_NODE2VEC 1
+#define PGLB_WALK_NODE2VEC_PLUS 2
+#define PGLB_WALK_MAX_REJECT 32
+#define PGLB_WALK_WORDS_PER_STEP 128
+/* Device.  Ids of `nodes` outside [0, N) give a row of -1 (callers are expected to reject them first). */
+int pglb_random_walk(const int64_t *indptr, const int64_t *cols, int64_t N, const int64_t *nodes, int64_t n,
+                     int64_t steps, int mode, double p, double q, uint64_t seed, int64_t *out, int64_t ldo,
+                     void *stream);
+/* Host twin: the same arguments on host pointers, blocking.  An id outside [0, N) is PGLB_ESHAPE. */
+int pglb_random_walk_host(const int64_t *indptr, const int64_t *cols, int64_t N, const int64_t *nodes, int64_t n,
+                          int64_t steps, int mode, double p, double q, uint64_t seed, int64_t *out, int64_t ldo);
+/* Skip-gram pairs of walks[n, W] (row stride ldw; a walk is the entries before its row's first -1).
+ * Position i of walk w < n draws r = 1 + umul64hi(mix64(mix64(seed ^ mix64(w)) + i), win_size) and pairs
+ * (walk[i], walk[j]) for every j in [i - r, i + r] inside the walk with walk[j] != walk[i], in that order.
+ *   count: offsets[n*W + 1]; offsets[p + 1] - offsets[p] = pairs of position p = w*W + i, offsets[n*W] = total.
+ *   fill : src[total], dst[total] in walk, position, j order.
+ * ws: pglb_skip_gram_ws bytes, the same buffer passed to both calls, untouched between them. */
+int pglb_skip_gram_ws(int64_t n, int64_t W, size_t *ws_bytes);
+int pglb_skip_gram_count(const int64_t *walks, int64_t n, int64_t W, int64_t ldw, int64_t win_size, uint64_t seed,
+                         int64_t *offsets, void *ws, size_t ws_bytes, void *stream);
+int pglb_skip_gram_fill(const int64_t *walks, int64_t n, int64_t W, int64_t ldw, int64_t win_size, uint64_t seed,
+                        const int64_t *offsets, int64_t *src, int64_t *dst, void *ws, size_t ws_bytes,
+                        void *stream);
+
 /* Same contract as pglb_memcpy2d_async, but the copy is done by a kernel through the unified address
  * space (zero-copy loads / stores across PCIe; the host side must be pinned memory).  For narrow column
  * blocks, where the copy engine's 2-D transfers run at about half the PCIe rate.  width, pitches and both

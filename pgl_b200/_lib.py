@@ -2,7 +2,7 @@
 shared library is missing this module raises at import time."""
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_int, c_int64, c_size_t, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_int, c_int64, c_size_t, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PGLB_LIB") or os.path.join(_HERE, "libpglb.so")
@@ -13,6 +13,7 @@ PGLB_CUDA_ERR_BASE = 1000
 REDUCE = {"sum": 0, "mean": 1, "max": 2, "min": 3}
 MSG = {"copy": 0, "add": 1, "sub": 2, "mul": 3, "div": 4}
 BCAST_FULL, BCAST_HEAD, BCAST_SCALAR = 0, 1, 2
+WALK_UNIFORM, WALK_NODE2VEC, WALK_NODE2VEC_PLUS = 0, 1, 2
 
 
 class PglbError(RuntimeError):
@@ -91,6 +92,11 @@ _SIGS = {
     "pglb_halo_plan_count": (c_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _p, c_size_t, _p]),
     "pglb_halo_plan_fill": (c_int, [_p, _i64, _i64, _i64, _i64, _p, _i64, _p, _p, _p, _p, _p, _p, c_size_t, _p]),
     "pglb_metis_partition": (c_int, [c_char_p, _i64, _p, _p, _i64, _p, _p, c_int, _p]),
+    "pglb_random_walk": (c_int, [_p, _p, _i64, _p, _i64, _i64, c_int, c_double, c_double, c_uint64, _p, _i64, _p]),
+    "pglb_random_walk_host": (c_int, [_p, _p, _i64, _p, _i64, _i64, c_int, c_double, c_double, c_uint64, _p, _i64]),
+    "pglb_skip_gram_ws": (c_int, [_i64, _i64, POINTER(c_size_t)]),
+    "pglb_skip_gram_count": (c_int, [_p, _i64, _i64, _i64, _i64, c_uint64, _p, _p, c_size_t, _p]),
+    "pglb_skip_gram_fill": (c_int, [_p, _i64, _i64, _i64, _i64, c_uint64, _p, _p, _p, _p, c_size_t, _p]),
 }
 
 for _name, (_res, _args) in _SIGS.items():

@@ -14,9 +14,8 @@
 // owns a `table` of num_nodes int64 filled with INT64_MAX; the call leaves it filled with INT64_MAX
 // again (only touched entries are reset), so it is allocated once per graph.
 //
-// STATUS: written after round 1's GPU budget was spent -- compiles for sm_100a, host logic and the
-// CPU restatement are tested, NOT yet run on hardware (tests/test_gpu_sampling.py is gated behind
-// PGLB_EXPERIMENTAL=1).
+// Runs on hardware and is tested there (tests/test_gpu_sampling.py, DESIGN.md section 4.11); the CPU restatement of
+// both kernels is tests/test_sampling_model.py.
 #include <limits.h>
 
 #include "common.cuh"

@@ -20,7 +20,7 @@ import torch
 from . import ops
 from .message import Message
 from .utils import op
-from .utils.edge_index import EdgeIndex
+from .utils.edge_index import EdgeIndex, sorted_successor_csr
 from .utils.helper import (check_is_tensor, generate_segment_id_from_index, maybe_num_nodes,
                            to_tensor)
 
@@ -140,7 +140,7 @@ class Graph(object):
                 if isinstance(ng, np.ndarray):
                     self._num_graph = int(ng.reshape(-1)[0])
             self._nodes = None
-            for a in ("_dst_uniq_ind", "_dst_segment_ids", "_src_uniq_ind", "_src_segment_ids"):
+            for a in ("_dst_uniq_ind", "_dst_segment_ids", "_src_uniq_ind", "_src_segment_ids", "_succ_csr"):
                 self.__dict__.pop(a, None)
             return self
         num_nodes = new["_num_nodes"] if to_t else int(self._n)
@@ -558,6 +558,14 @@ class Graph(object):
             self._adj_src_index = EdgeIndex.from_edges(
                 u=self._edges[:, 0], v=self._edges[:, 1], num_nodes=self._num_nodes, v_bound=self._n)
         return self._adj_src_index
+
+    def successor_csr(self):
+        """(indptr, cols) of the successors with every row in ascending order (cached): what the random walks of
+        pgl_b200.sampling read, where "is x a successor of v" is a binary search.  indptr is adj_src_index's."""
+        csr = self.__dict__.get("_succ_csr")
+        if csr is None:
+            csr = self._succ_csr = sorted_successor_csr(self._edges[:, 0], self._edges[:, 1], self._n)
+        return csr
 
     @property
     def adj_dst_index(self):

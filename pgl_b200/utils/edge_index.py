@@ -47,6 +47,20 @@ def build_index_host(u, v, num_nodes):
     return degree, sv, su, se, indptr
 
 
+def sorted_successor_csr(u, v, num_nodes):
+    """(indptr, cols) keyed by ``u`` with every row's ``v`` in ascending order: the stable index build keyed by
+    ``v``, then again keyed by ``u``.  indptr is the one of ``EdgeIndex.from_edges(u, v)``.  Host or device, as the
+    inputs are."""
+    if check_is_tensor(u, v):
+        n = int(num_nodes.item()) if isinstance(num_nodes, torch.Tensor) else int(num_nodes)
+        _, by_v_u, by_v_v, _, _ = ops.csr_build(v, u, n)
+        _, cols, _, _, indptr = ops.csr_build(by_v_u, by_v_v, n)
+    else:
+        _, by_v_u, by_v_v, _, _ = build_index_host(v, u, num_nodes)
+        _, cols, _, _, indptr = build_index_host(by_v_u, by_v_v, num_nodes)
+    return indptr, cols
+
+
 class EdgeIndex(object):
     """Sorted edges in compressed form, keyed by ``u`` (reference edge_index.py:27-36)."""
 
